@@ -2,6 +2,7 @@
 """Benchmark of the message-passing hot path (BASELINE.json metric: edges/sec per GNN layer; % of HBM roofline).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--agg sum|max] [--workload graph2class|varmisuse]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload (BASELINE.json configs[1]): Graph2Class synthetic batch -- 80 graphs x 2,560 nodes = 204,800 nodes, 8 raw
@@ -13,6 +14,9 @@ Multi-GPU: graph-granular sharding -- every rank owns its own batch of graphs (b
 data-path collective), weak scaling; value = (all ranks' edges) * L / max-over-ranks time.
 `--impl reference`: the reference's CPU path (torch-CPU oracle port: same ATen ops as the reference classes + the
 restated torch_scatter) on all host threads, rank 0 only.
+`--dump-outputs DIR`: after the timed steps, rank 0 writes the output node states of the last timed step of the headline loop
+to DIR/node_states.npy (float32; a fixed, seeded sample of DUMP_MAX_ROWS rows when there are more).  The inputs and
+parameters are seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -30,6 +34,7 @@ sys.path.insert(0, ROOT)
 HIDDEN = 128
 NUM_LAYERS = 8
 L2_BYTES = 126e6
+DUMP_MAX_ROWS = 65536          # 32 MiB of fp32 states at HIDDEN = 128
 
 
 def measured_peaks():
@@ -293,6 +298,19 @@ def cpu_reference_run(batch, gnn, agg: str, steps: int, warmup: int, budget_s: f
     }
 
 
+def dump_outputs(out_dir: str, node_states: torch.Tensor) -> None:
+    """Writes `node_states` ([N, HIDDEN], any float dtype, on the GPU) as out_dir/node_states.npy in float32: all rows, or the
+    same seeded sample of DUMP_MAX_ROWS rows (in ascending row order) on every run when N is larger."""
+    import numpy as np
+
+    n = node_states.shape[0]
+    if n > DUMP_MAX_ROWS:
+        rows = torch.randperm(n, generator=torch.Generator().manual_seed(0))[:DUMP_MAX_ROWS].sort().values
+        node_states = node_states.index_select(0, rows.to(node_states.device))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "node_states.npy"), node_states.float().cpu().numpy())
+
+
 # ------------------------------------------------------------------------------------------------------
 def main():
     ap = argparse.ArgumentParser()
@@ -311,7 +329,13 @@ def main():
     ap.add_argument("--no-train", action="store_true", help="skip the forward + backward extra measurement")
     ap.add_argument("--no-row-shard", action="store_true", help="skip the node-range-split (all-gather) extra measurement")
     ap.add_argument("--profile", action="store_true", help="only the HBM-resident loop (for runs under ncu); prints no bench line")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the output node states of the last timed step to DIR/node_states.npy (see the module docstring)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.profile):
+        ap.error("--dump-outputs applies to the timed GPU loop (--impl ours, without --profile)")
     args.warmup = max(args.warmup, 3)
     if args.layers == "mlp":
         args.no_cpu_baseline = True      # the CPU-port leg is written for the headline (gated) stack
@@ -474,7 +498,7 @@ def main():
             dist.barrier()
         torch.cuda.synchronize()
 
-    def timed(fn, steps, warmup, finish=None):
+    def timed(fn, steps, warmup, finish=None, keep_last=False):
         for _ in range(warmup):
             fn()
         if finish:
@@ -484,12 +508,14 @@ def main():
         a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         a.record()
         t_host = time.perf_counter()
-        for _ in range(steps):
+        for _ in range(steps - 1):
             fn()
+        last = fn()
         if finish:
             finish()
         b.record()
         timed.host_ms = (time.perf_counter() - t_host) * 1e3 / steps   # host enqueue time per step (no device sync)
+        timed.last = last if keep_last else None                         # what the last timed step returned
         barrier()
         ms = a.elapsed_time(b)
         t = torch.tensor([ms], device=dev)
@@ -503,8 +529,11 @@ def main():
         torch.cuda.synchronize()
         return
     with ClockSampler(local_rank) as clocks:
-        ms_step, launches = timed(step_resident, args.steps, args.warmup)
+        ms_step, launches = timed(step_resident, args.steps, args.warmup, keep_last=bool(args.dump_outputs))
     clock_summary = clocks.summary()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, timed.last)
+    timed.last = None
     ms_e2e_serial, _ = timed(step_e2e, args.steps, args.warmup)
     pipe = PipelinedE2E()
     ms_e2e_eager, _ = timed(pipe.step, args.steps, args.warmup, finish=pipe.finish)
@@ -541,10 +570,10 @@ def main():
 
     # ---- per-kernel timing leg (CUDA events on the launch stream, inside the library) -> roofline
     N.kernel_timing(True)
-    for _ in range(3):
+    for _ in range(args.warmup):
         step_resident()
     N.read_kernel_timing()
-    ksteps = max(3, min(args.steps, 10))
+    ksteps = args.steps
     for _ in range(ksteps):
         step_resident()
     kt = N.read_kernel_timing()
@@ -699,7 +728,7 @@ def main():
                 out = gnn.gnn(h_train, adj, None, n2g, {}, {})
                 out.mean().backward()
 
-            ms_train, _ = timed(step_train, max(3, args.steps // 4), 2)
+            ms_train, _ = timed(step_train, args.steps, args.warmup)
             train = {"ms_per_step": ms_train, "value": E * NUM_LAYERS / (ms_train * 1e-3), "unit": "edges/s (forward + backward)",
                      "note": "fp32; forward = the fused kernels, backward = native edge-sized kernels on the transposed graph + library GEMMs "
                              "for the parameter gradients (ptgnn_b200/autograd.py)"}
